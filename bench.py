@@ -12,9 +12,12 @@ One "step" = one pass of the hot path over one batch of synthetic images:
                      (dsrg_b200/shard.py), each rank works through its shard in batches of 64: STRONG scaling.
                      The default (dsrg321) line also carries a `sweep4096` object measured in the same run.
 
-`python bench.py --gpus N --steps K --warmup W` prints ONE JSON line (rank 0).  Under torchrun
-(WORLD_SIZE > 1) every rank runs the same per-rank batch on its own GPU (images shard with no
-data-path collective; weak scaling) and the time is the max over ranks.
+`python bench.py --gpus N --steps K --warmup W` prints ONE JSON line (rank 0); the headline and `e2e` numbers
+each time exactly K steps.  Under torchrun (WORLD_SIZE > 1) every rank runs the same per-rank batch on its own
+GPU (images shard with no data-path collective; weak scaling) and the time is the max over ranks.
+
+`--dump-outputs DIR` also writes what the timed path computed in its last timed step (rank 0's buffers) as
+DIR/<name>.npy.  The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 `--impl reference` times the reference's CPU path instead (oracle port: oracle/crf_oracle.c +
 oracle/srg_oracle.py:srg_faithful) on all host cores; this and the `cpu_baseline` leg are the only
@@ -159,6 +162,24 @@ def usable_cpus():
     except Exception:
         pass
     return n
+
+
+DUMP_MAX_ELEMENTS = 1 << 22   # per array: 16 MB of float32, so the at most three arrays of a workload stay under 64 MB
+
+
+def dump_outputs(directory, arrays):
+    """Write each device tensor of ``arrays`` as directory/<name>.npy in float32 (float64 stays float64).  An array
+    of more than DUMP_MAX_ELEMENTS elements is written as a sample of its flattened elements: the sorted distinct
+    positions of DUMP_MAX_ELEMENTS draws of RandomState(0), the same in every run for the same shape."""
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMENTS:
+            pos = np.unique(np.random.RandomState(0).randint(0, t.numel(), DUMP_MAX_ELEMENTS))
+            t = t.reshape(-1)[torch.from_numpy(pos).to(t.device)]
+        a = t.cpu().numpy()
+        np.save(os.path.join(directory, name + ".npy"), a.astype(np.float64 if a.dtype == np.float64 else np.float32))
 
 
 def synth_batch(H, W, B, unique=8):
@@ -349,17 +370,18 @@ def run_b200(args, rank, local_rank, world):
     if sampler:
         torch.cuda.synchronize()
         sampler.mark()
-    # EXACTLY K steps per timed block (barrier + synchronize on both sides, max over ranks).  A block of the default
-    # K is a fraction of a second, so the block is repeated until ~1.5 s of GPU time has been sampled (at most 9
-    # blocks) and the MEDIAN block is reported: the number does not hang on one quarter-second window and the clock
-    # sampler sees dozens of samples under load.
-    trials = [timed(step, args.steps)]
-    while len(trials) < 9 and sum(trials) < 1500.0:
-        trials.append(timed(step, args.steps))
+    # exactly --steps timed steps, one block (barrier + synchronize on both sides, max over ranks)
+    ms = timed(step, args.steps)
     clocks = sampler.stop() if sampler else None
-    launches = eng.take_launch_count() // len(trials)
-    ms = float(np.median(trials))
+    launches = eng.take_launch_count()
     value = images_per_step * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # what a caller of the timed path holds after its last step (dsrg_forward_dev also clamps probs in place);
+        # taken before the legs below reuse the buffers
+        outs = {"crf": {"crf_marginals": d_q}, "srg": {"seeds": d_seeds}}.get(what, {"seeds": d_seeds, "probs": d_probs})
+        if "loss" in what:
+            outs["loss_terms"] = d_terms
+        dump_outputs(args.dump_outputs, outs)
 
     # per-kernel durations by CUDA events on the launching stream, same K steps repeated
     eng.profile(True)
@@ -449,12 +471,8 @@ def run_b200(args, rank, local_rank, world):
                 dist.all_reduce(t, op=dist.ReduceOp.MAX)
                 dt = float(t.item())
             return dt
-        dts = [host_block()]
-        while len(dts) < 7 and sum(dts) < 1.5 and not sweep:
-            dts.append(host_block())
-        dt = float(np.median(dts))
+        dt = host_block()
         e2e = {"value": images_per_step * args.steps / dt, "unit": "images/s", "h2d_bytes_per_step": int(h2d),
-               "timed_blocks": len(dts),
                "d2h_bytes_per_step": int(d2h), "api": "dsrg_*_host (C ABI, pinned host buffers)",
                "note": "inputs are re-sent from the same pinned buffers every step; the in-place 1e-4 clamp of probs "
                        "(pylayers.py:312) therefore only changes values during the first warm-up step"}
@@ -560,8 +578,6 @@ def run_b200(args, rank, local_rank, world):
                        "thresholds": [TH1, TH2], "images": "%s, cam-like cues, 8 distinct images repeated" % IMAGE_VARIANT,
                        "l2": "inputs larger than L2 (%.0f MB of probs+cues per step)" % (2 * 4 * M * N * B / 1e6),
                        "parallelism": "dp%d (images shard, no data-path collective)" % world},
-            "timed_blocks": {"n": len(trials), "steps_each": args.steps, "ms_per_step": [round(t / args.steps, 4) for t in trials],
-                             "reported": "median block"},
             "clocks": clocks, "e2e": e2e, "gpu_launches": int(launches), "roofline": roofline,
             "kernels": kernels, "cpu_baseline": cpu_baseline, **extras,
         }))
@@ -604,7 +620,12 @@ def main():
     ap.add_argument("--images", default="smooth", choices=["smooth", "photo", "noise"],
                     help="synthetic image variant: smooth (headline), photo (1/f spectrum) or uniform noise (worst "
                          "case: every tile overflows the shared-memory path)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (a fixed sample of large arrays, "
+                         "64 MB at most)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
     global IMAGE_VARIANT
     IMAGE_VARIANT = args.images
     claim_stdout()

@@ -6,8 +6,8 @@ BalancedSeedLossLayer, ConstrainLossLayer and AnnotationLayer are pulled out of
 needs caffe, theano and cPickle at import time; nothing is copied) and executed against
 ``oracle/theano_shim`` (the Theano stand-in) and a minimal Blob/Layer stand-in for pycaffe.  The outputs
 are what pins ``oracle/loss_oracle.py`` and ``oracle/annot_oracle.py``: tests/golden/make_golden.py
-freezes them in tests/golden/layers_ref.npz, and tests/test_oracle_golden.py compares live when the
-reference is mounted.
+freezes them in tests/golden/layers_ref.npz and layers_ref_sweep.npz, which tests/test_oracle_golden.py
+compares against.
 """
 import ast
 import os

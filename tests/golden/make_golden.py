@@ -14,8 +14,17 @@ Runs ONLY in the dev container (needs /root/reference):
   * CRF: oracle/crf_oracle.c marginals (restatement; its lattice is pinned by the previous
     item) -> tests/golden/crf_oracle_*.npz, so GPU runs have a frozen target even if the
     oracle sources change later.
+  * the reference's own code on further seeded inputs, so that the tests compare the restatements
+    with it without the reference at hand:
+      srg_sweep      generate_seed_step on six random problems -> srg_ref_sweep.npz (packed bits)
+      lattice_random permutohedral.cpp on three random feature matrices -> lattice_ref_random.npz
+      crf_ref        the compiled CRF sources (oracle/_ref/libdensecrf_ref.so) -> crf_ref_build.npz:
+                     sha256 of the marginals / MAP labels, bit-exact targets of the restatement
+      layers_sweep   the loss layer classes on three more shapes -> layers_ref_sweep.npz (float64,
+                     a fixed sample of each gradient)
 
-usage: python tests/golden/make_golden.py [srg lattice crf post layers]   (default: all)
+usage: python tests/golden/make_golden.py [srg lattice crf post layers srg_sweep lattice_random crf_ref layers_sweep]
+       (default: all)
 """
 import hashlib
 import os
@@ -218,9 +227,160 @@ def make_layers():
     np.savez_compressed(os.path.join(OUT, "layers_ref.npz"), **rec)
 
 
+SRG_SWEEP = [(500 + i, 19 + 3 * i, 31 - 2 * i, ["cam", "random"][i % 2]) for i in range(6)]  # index, H, W, cues
+
+
+def srg_sweep_inputs(index, H, W, cues):
+    p = synth.make_problem(index, H, W, cues=cues, image="noise")
+    return p["labels"], p["cues"], p["probs"]
+
+
+def make_srg_sweep():
+    rec = {}
+    for k, case in enumerate(SRG_SWEEP):
+        labels, cu, probs = srg_sweep_inputs(*case)
+        out = srg_oracle.run_reference(labels, cu, probs, 0.99, 0.85)
+        rec["%d/inputs_sha256" % k] = digest(labels, cu, probs)
+        rec["%d/seeds_bits" % k], rec["%d/seeds_shape" % k] = np.packbits(out.astype(np.uint8)), np.array(out.shape)
+        print("srg sweep", case, int(cu.sum()), "->", int(out.sum()))
+    np.savez_compressed(os.path.join(OUT, "srg_ref_sweep.npz"), **rec)
+
+
+LATTICE_FIELDS = ("offset", "bary", "rank", "n1", "n2")
+
+
+def lattice_random_inputs():
+    """(features, values) pairs: random 2-d (spatial) and 5-d (bilateral) feature matrices, 21 values per point."""
+    rng = np.random.RandomState(3)
+    cases = []
+    for H, W, d in ((23, 31, 2), (23, 31, 5), (40, 17, 5)):
+        f = (rng.rand(H * W, d) * [3, 3, 19, 19, 19][:d]).astype(np.float32)
+        cases.append((f, rng.rand(H * W, 21).astype(np.float32)))
+    return cases
+
+
+def make_lattice_random():
+    rec = {}
+    for k, (f, x) in enumerate(lattice_random_inputs()):
+        L = crf_oracle.RefLattice(f)
+        rec["%d/inputs_sha256" % k] = digest(f, x)
+        rec["%d/M" % k] = L.M
+        for name in LATTICE_FIELDS:
+            rec["%d/sha_%s" % (k, name)] = digest(getattr(L, name))
+        rec["%d/sha_compute" % k] = digest(L.compute(x, "dispatch"))
+        print("lattice random", k, f.shape, "M", L.M)
+    np.savez_compressed(os.path.join(OUT, "lattice_ref_random.npz"), **rec)
+
+
+CRF_REF_ITERS = (0, 1, 4)
+CRF_REF_SHAPES = [(97, 131, 21, 1.0, "smooth"), (60, 45, 5, 12.0, "noise"), (33, 33, 2, 1.0, "noise"),  # H, W, M, sf, image
+                  (161, 161, 21, 1.0, "smooth"), (120, 90, 21, 1.0, "photo")]
+CRF_DIRECT_CASES = [(41, 41, 12.0, "smooth"), (97, 131, 1.0, "smooth"), (64, 64, 1.0, "noise")]  # H, W, sf, image
+
+
+def crf_shape_key(H, W, M, sf, img):
+    return "shape_%d_%d_%d_%g_%s" % (H, W, M, sf, img)
+
+
+def crf_shape_inputs(H, W, M, img):
+    """(image, [log-probability unary, probability unary])."""
+    rng = np.random.RandomState(H * 7 + M)
+    im = synth.make_image(rng, H, W, img)
+    logits = rng.randn(H, W, M) * 2
+    logits[H // 4: H // 2, W // 3:, 0] += 4
+    e = np.exp(logits - logits.max(2, keepdims=True))
+    pr = (e / e.sum(2, keepdims=True)).astype(np.float32)
+    pr[pr < 1e-5] = 1e-5
+    return im, [np.log(pr), pr]
+
+
+def crf_direct_key(H, W):
+    return "direct_%dx%d" % (H, W)
+
+
+def crf_direct_inputs(H, W, sf, img):
+    """(image, unary) of the GPU test against the reference build: probabilities at scale_factor 12, else log p."""
+    p = synth.make_problem(950 + H, H, W, image=img)
+    pr = np.transpose(p["probs"], (1, 2, 0)).copy()
+    pr[pr < 1e-5] = 1e-5
+    return p["image"], pr if sf > 1 else np.log(pr)
+
+
+def crf_objects(cls, im, unary, sf):
+    """A DenseCRF-like object of class ``cls`` set up the way CRF.py:21-33 does."""
+    H, W, M = unary.shape
+    c = cls(W, H, M)
+    c.set_unary_energy(-unary.ravel())
+    c.add_pairwise_energy(10, 80 / sf, 80 / sf, 13, 13, 13, 3, 3 / sf, 3 / sf, im.ravel())
+    return c
+
+
+def make_crf_ref():
+    rec = {}
+    for i, (name, H, W, var, sf, kind) in enumerate(CRF_CASES):
+        im, unary = crf_inputs(H, W, var, kind, i)
+        rec[name + "/inputs_sha256"] = digest(im, unary)
+        rec[name + "/crf"] = digest(crf_oracle.CRF_reference(im, unary, 10, sf))
+        r = crf_objects(crf_oracle.RefDenseCRF, im, unary, sf)
+        for it in CRF_REF_ITERS:
+            rec["%s/inference%d" % (name, it)] = digest(r.inference(it))
+            rec["%s/map%d" % (name, it)] = digest(r.map(it))
+    for H, W, M, sf, img in CRF_REF_SHAPES:
+        im, unaries = crf_shape_inputs(H, W, M, img)
+        key = crf_shape_key(H, W, M, sf, img)
+        rec[key + "/inputs_sha256"] = digest(im, *unaries)
+        for kind, unary in zip(("logp", "p"), unaries):
+            rec["%s/%s" % (key, kind)] = digest(crf_oracle.CRF_reference(im, unary, 10, sf, color_factor=13))
+    for H, W, sf, img in CRF_DIRECT_CASES:
+        im, unary = crf_direct_inputs(H, W, sf, img)
+        key = crf_direct_key(H, W)
+        rec[key + "/inputs_sha256"] = digest(im, unary)
+        rec[key + "/crf"] = digest(crf_oracle.CRF_reference(im, unary, 10, sf))
+        rec[key + "/map"] = digest(crf_objects(crf_oracle.RefDenseCRF, im, unary, sf).map(10))
+    print("crf ref", len(rec), "digests")
+    np.savez_compressed(os.path.join(OUT, "crf_ref_build.npz"), **rec)
+
+
+LAYER_SWEEP_SEEDS = (5, 6, 7)
+LAYER_SAMPLE = 512   # elements kept of each gradient array (float64; the whole array would exceed what a fixture needs)
+
+
+def layer_sweep_inputs(seed):
+    return layer_inputs(seed, N=2 + seed % 3, H=5 + seed, W=11 - seed)
+
+
+def layer_sample(a, seed):
+    """A fixed, seeded sample of the flattened array ``a`` (all of it when it is small)."""
+    a = np.ravel(a)
+    if a.size <= LAYER_SAMPLE:
+        return a
+    return a[np.sort(np.random.RandomState(seed).choice(a.size, LAYER_SAMPLE, replace=False))]
+
+
+def make_layers_sweep():
+    from oracle import ref_layers
+    rec = {}
+    for seed in LAYER_SWEEP_SEEDS:
+        logits, p, lab, td, ls = layer_sweep_inputs(seed)
+        k = "s%d_" % seed
+        rec[k + "inputs_sha256"] = digest(logits, p, lab, td, ls)
+        loss, grad = ref_layers.balanced_seed_loss_layer(p, lab, "float64")
+        pr, gd = ref_layers.softmax_layer(logits, td, "float64")
+        cl, g0, g1 = ref_layers.constrain_loss_layer(p, ls, "float64")
+        rec[k + "seed_loss"], rec[k + "constrain_loss"] = loss, cl
+        for name, a in (("seed_grad", grad), ("softmax_probs", pr), ("softmax_grad", gd), ("constrain_g0", g0),
+                        ("constrain_g1", g1)):
+            rec[k + name] = layer_sample(a, seed)
+        print("layers sweep seed", seed, float(loss), float(cl))
+    np.savez_compressed(os.path.join(OUT, "layers_ref_sweep.npz"), **rec)
+
+
 if __name__ == "__main__":
-    assert srg_oracle.reference_available(), "needs /root/reference"
-    what = sys.argv[1:] or ["srg", "lattice", "crf", "post", "layers"]
+    assert srg_oracle.reference_available(), "needs the reference checkout (oracle/srg_oracle.py:REF_ROOT)"
+    what = sys.argv[1:] or ["srg", "lattice", "crf", "post", "layers", "srg_sweep", "lattice_random", "crf_ref",
+                            "layers_sweep"]
     crf_oracle.build(force=True)
     for w in what:
-        {"srg": make_srg, "lattice": make_lattice, "crf": make_crf, "post": make_post, "layers": make_layers}[w]()
+        {"srg": make_srg, "lattice": make_lattice, "crf": make_crf, "post": make_post, "layers": make_layers,
+         "srg_sweep": make_srg_sweep, "lattice_random": make_lattice_random, "crf_ref": make_crf_ref,
+         "layers_sweep": make_layers_sweep}[w]()

@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 
 from conftest import load_golden
-from helpers import crf_case_inputs, make_golden
+from helpers import crf_case_inputs, digest, make_golden
 from dsrg_b200 import api, synth
 from oracle import crf_oracle
 
@@ -290,25 +290,23 @@ def test_densecrf_objects_share_one_engine(torch_cuda):
     assert np.isfinite(got).all()
 
 
-@pytest.mark.skipif(not crf_oracle.ref_crf_available(), reason="oracle/_ref/libdensecrf_ref.so was not shipped")
-@pytest.mark.parametrize("H,W,sf,img", [(41, 41, 12.0, "smooth"), (97, 131, 1.0, "smooth"), (64, 64, 1.0, "noise")])
+@pytest.mark.parametrize("H,W,sf,img", make_golden.CRF_DIRECT_CASES)
 def test_crf_against_the_reference_build_directly(torch_cuda, H, W, sf, img):
-    """CUDA path vs the reference's OWN CRF sources (compiled unmodified into oracle/_ref, oracle/Makefile):
-    marginals within 1e-4, MAP labels equal except at near-ties."""
-    p = synth.make_problem(950 + H, H, W, image=img)
-    pr = np.transpose(p["probs"], (1, 2, 0)).copy()
-    pr[pr < 1e-5] = 1e-5
-    unary = pr if sf > 1 else np.log(pr)
-    want = crf_oracle.CRF_reference(p["image"], unary, 10, sf)
+    """CUDA path vs the reference's OWN CRF sources (compiled unmodified, oracle/Makefile): marginals within 1e-4,
+    MAP labels equal except at near-ties.  The reference build's outputs are the C restatement's, bit for bit:
+    the digests of that build's outputs in crf_ref_build.npz say so for these very inputs."""
+    g = load_golden("crf_ref_build.npz")
+    key = make_golden.crf_direct_key(H, W)
+    im, unary = make_golden.crf_direct_inputs(H, W, sf, img)
+    assert digest(im, unary) == str(g[key + "/inputs_sha256"])
+    want = crf_oracle.CRF(im, unary, 10, sf)
+    assert digest(want) == str(g[key + "/crf"]), "the restatement no longer reproduces the reference build"
     eng = api.Engine(1, H, W, 21)
-    got = eng.crf_host(unary[None], p["image"][None], api.crf_params(sf))[0]
+    got = eng.crf_host(unary[None], im[None], api.crf_params(sf))[0]
     assert np.abs(got - want).max() <= 1e-4
-    ref = crf_oracle.RefDenseCRF(W, H, 21)
-    ours = api.DenseCRF(W, H, 21)
-    for c in (ref, ours):
-        c.set_unary_energy(-unary.ravel())
-        c.add_pairwise_energy(10, 80 / sf, 80 / sf, 13, 13, 13, 3, 3 / sf, 3 / sf, p["image"].ravel())
-    a, b = ours.map(10), ref.map(10)
+    b = make_golden.crf_objects(crf_oracle.DenseCRF, im, unary, sf).map(10)
+    assert digest(b) == str(g[key + "/map"]), "the restatement no longer reproduces the reference build"
+    a = make_golden.crf_objects(api.DenseCRF, im, unary, sf).map(10)
     bad = a != b
     if bad.any():
         top2 = np.sort(want.reshape(-1, 21), axis=1)[:, -2:]

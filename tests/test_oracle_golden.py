@@ -4,7 +4,6 @@ import numpy as np
 import pytest
 
 from conftest import load_golden
-from dsrg_b200 import synth
 from helpers import crf_case_inputs, digest, make_golden, srg_case_inputs
 from oracle import crf_oracle, loss_oracle, srg_oracle
 
@@ -30,14 +29,16 @@ def test_srg_faithful_port_matches_reference_golden(name):
     assert np.array_equal(got, want)
 
 
-@pytest.mark.skipif(not srg_oracle.reference_available(), reason="needs /root/reference (dev container)")
 def test_srg_reference_in_place_random_sweep():
-    from dsrg_b200 import synth
-    for i in range(6):
-        p = synth.make_problem(500 + i, 19 + 3 * i, 31 - 2 * i, cues=["cam", "random"][i % 2], image="noise")
-        want = srg_oracle.run_reference(p["labels"], p["cues"], p["probs"], 0.99, 0.85)
-        assert np.array_equal(srg_oracle.srg_closed_form(p["labels"], p["cues"], p["probs"], 0.99, 0.85), want)
-        assert np.array_equal(srg_oracle.srg_faithful(p["labels"], p["cues"], p["probs"], 0.99, 0.85), want)
+    """Both restatements against the reference's own generate_seed_step on six random problems (srg_ref_sweep.npz)."""
+    g = load_golden("srg_ref_sweep.npz")
+    for k, case in enumerate(make_golden.SRG_SWEEP):
+        labels, cues, probs = make_golden.srg_sweep_inputs(*case)
+        assert digest(labels, cues, probs) == str(g["%d/inputs_sha256" % k]), "synthetic generator drifted"
+        shape = g["%d/seeds_shape" % k]
+        want = np.unpackbits(g["%d/seeds_bits" % k])[: int(np.prod(shape))].reshape(shape).astype(np.float32)
+        assert np.array_equal(srg_oracle.srg_closed_form(labels, cues, probs, 0.99, 0.85), want)
+        assert np.array_equal(srg_oracle.srg_faithful(labels, cues, probs, 0.99, 0.85), want)
 
 
 @pytest.mark.parametrize("case", make_golden.LATTICE_CASES, ids=[c[0] for c in make_golden.LATTICE_CASES])
@@ -57,17 +58,17 @@ def test_oracle_lattice_matches_reference_permutohedral_golden(case):
     np.testing.assert_allclose(L.bary.sum(1), 1.0, atol=2e-6)  # barycentric weights sum to one
 
 
-@pytest.mark.skipif(not crf_oracle.ref_available(), reason="oracle/_ref not built")
 def test_oracle_lattice_bit_exact_vs_ref_so_live():
-    rng = np.random.RandomState(3)
-    for H, W, d in ((23, 31, 2), (23, 31, 5), (40, 17, 5)):
-        f = (rng.rand(H * W, d) * [3, 3, 19, 19, 19][:d]).astype(np.float32)
-        a, b = crf_oracle.OracleLattice(f), crf_oracle.RefLattice(f)
-        assert a.M == b.M
-        for k in ("offset", "bary", "rank", "n1", "n2"):
-            assert np.array_equal(getattr(a, k), getattr(b, k)), k
-        x = rng.rand(H * W, 21).astype(np.float32)
-        assert np.array_equal(a.compute(x, "sse"), b.compute(x, "dispatch"))
+    """oracle/crf_oracle.c lattice vs the digests of the reference's own permutohedral.cpp (lattice_ref_random.npz)
+    on random feature matrices: every structure array and the dispatching compute() bit for bit."""
+    g = load_golden("lattice_ref_random.npz")
+    for k, (f, x) in enumerate(make_golden.lattice_random_inputs()):
+        assert digest(f, x) == str(g["%d/inputs_sha256" % k]), "input generator drifted"
+        a = crf_oracle.OracleLattice(f)
+        assert a.M == int(g["%d/M" % k])
+        for name in make_golden.LATTICE_FIELDS:
+            assert digest(getattr(a, name)) == str(g["%d/sha_%s" % (k, name)]), name
+        assert digest(a.compute(x, "sse")) == str(g["%d/sha_compute" % k])
 
 
 @pytest.mark.parametrize("name", [c[0] for c in make_golden.CRF_CASES])
@@ -154,43 +155,30 @@ def test_post_oracle_matches_frozen_golden(case):
     assert np.array_equal(lab0, p0.argmax(2)) and p0.min() >= np.float32(1e-5)
 
 
-needs_ref_crf = pytest.mark.skipif(not crf_oracle.ref_crf_available(),
-                                   reason="oracle/_ref/libdensecrf_ref.so not built (needs /root/reference once)")
-
-
-@needs_ref_crf
 @pytest.mark.parametrize("name", [c[0] for c in make_golden.CRF_CASES])
 def test_crf_oracle_is_bit_exact_vs_the_reference_build(name):
     """The C restatement against the reference's OWN CRF sources (densecrf.cpp, pairwise.cpp, ... compiled
-    unmodified, oracle/Makefile) through DenseCRFWrapper: marginals and MAP labels, several iteration counts."""
+    unmodified, oracle/Makefile) through DenseCRFWrapper: marginals and MAP labels, several iteration counts,
+    compared with the digests of that build's outputs (crf_ref_build.npz)."""
+    g = load_golden("crf_ref_build.npz")
     im, unary, sf = crf_case_inputs(name)
-    H, W, M = unary.shape
-    assert np.array_equal(crf_oracle.CRF(im, unary, 10, sf), crf_oracle.CRF_reference(im, unary, 10, sf))
-    o, r = crf_oracle.DenseCRF(W, H, M), crf_oracle.RefDenseCRF(W, H, M)
-    for c in (o, r):
-        c.set_unary_energy(-unary.ravel())
-        c.add_pairwise_energy(10, 80 / sf, 80 / sf, 13, 13, 13, 3, 3 / sf, 3 / sf, im.ravel())
-    for it in (0, 1, 4):
-        assert np.array_equal(o.inference(it), r.inference(it))
-        assert np.array_equal(o.map(it), r.map(it))
+    assert digest(im, unary) == str(g[name + "/inputs_sha256"])
+    assert digest(crf_oracle.CRF(im, unary, 10, sf)) == str(g[name + "/crf"])
+    o = make_golden.crf_objects(crf_oracle.DenseCRF, im, unary, sf)
+    for it in make_golden.CRF_REF_ITERS:
+        assert digest(o.inference(it)) == str(g["%s/inference%d" % (name, it)]), it
+        assert digest(o.map(it)) == str(g["%s/map%d" % (name, it)]), it
 
 
-@needs_ref_crf
-@pytest.mark.parametrize("H,W,M,sf,img", [(97, 131, 21, 1.0, "smooth"), (60, 45, 5, 12.0, "noise"), (33, 33, 2, 1.0, "noise"),
-                                          (161, 161, 21, 1.0, "smooth"), (120, 90, 21, 1.0, "photo")])
+@pytest.mark.parametrize("H,W,M,sf,img", make_golden.CRF_REF_SHAPES)
 def test_crf_oracle_vs_reference_build_other_shapes(H, W, M, sf, img):
     """incl. M = 2, where Permutohedral::compute takes the seqCompute branch (permutohedral.cpp:600-601)."""
-    rng = np.random.RandomState(H * 7 + M)
-    im = synth.make_image(rng, H, W, img)
-    logits = rng.randn(H, W, M) * 2
-    logits[H // 4: H // 2, W // 3:, 0] += 4
-    e = np.exp(logits - logits.max(2, keepdims=True))
-    pr = (e / e.sum(2, keepdims=True)).astype(np.float32)
-    pr[pr < 1e-5] = 1e-5
-    for unary in (np.log(pr), pr):
-        a = crf_oracle.CRF(im, unary, 10, sf, color_factor=13)
-        b = crf_oracle.CRF_reference(im, unary, 10, sf, color_factor=13)
-        assert np.array_equal(a, b)
+    g = load_golden("crf_ref_build.npz")
+    key = make_golden.crf_shape_key(H, W, M, sf, img)
+    im, unaries = make_golden.crf_shape_inputs(H, W, M, img)
+    assert digest(im, *unaries) == str(g[key + "/inputs_sha256"])
+    for kind, unary in zip(("logp", "p"), unaries):
+        assert digest(crf_oracle.CRF(im, unary, 10, sf, color_factor=13)) == str(g["%s/%s" % (key, kind)]), kind
 
 
 # ---- a12 / f1 / f4: the loss and annotation oracles against the reference's own layer classes -------------------
@@ -231,25 +219,24 @@ def test_annotation_oracle_matches_the_reference_layer_golden(mirror):
     assert np.array_equal(t0, g[k + "labels"]) and np.array_equal(t1, want1) and digest(t2) == str(g[k + "images_sha256"])
 
 
-def _ref_layers():
-    from oracle import ref_layers
-    return ref_layers
-
-
-@pytest.mark.skipif(not srg_oracle.reference_available(), reason="needs /root/reference (dev container)")
 def test_reference_layers_run_in_place_random_sweep():
-    """Live: the reference's own layer classes (through the Theano stand-in) against the restatements on fresh inputs."""
-    rl = _ref_layers()
-    for seed in (5, 6, 7):
-        logits, p, lab, td, ls = make_golden.layer_inputs(seed, N=2 + seed % 3, H=5 + seed, W=11 - seed)
-        loss, grad = rl.balanced_seed_loss_layer(p, lab, "float64")
-        np.testing.assert_allclose(loss, loss_oracle.balanced_seed_loss(p, lab), rtol=1e-12)
-        np.testing.assert_allclose(grad, loss_oracle.balanced_seed_loss_grad(p, lab), rtol=1e-12, atol=1e-15)
-        pr, gd = rl.softmax_layer(logits, td, "float64")
-        np.testing.assert_allclose(pr, loss_oracle.softmax_layer_forward(logits), rtol=1e-12)
-        np.testing.assert_allclose(gd, loss_oracle.softmax_layer_backward(logits, td), rtol=1e-10, atol=1e-15)
-        cl, g0, g1 = rl.constrain_loss_layer(p, ls, "float64")
-        np.testing.assert_allclose(cl, loss_oracle.constrain_loss(p, ls), rtol=1e-12)
+    """The reference's own layer classes (through the Theano stand-in) against the restatements on three more shapes:
+    losses in full, a fixed sample of every gradient (layers_ref_sweep.npz)."""
+    g = load_golden("layers_ref_sweep.npz")
+    for seed in make_golden.LAYER_SWEEP_SEEDS:
+        logits, p, lab, td, ls = make_golden.layer_sweep_inputs(seed)
+        k = "s%d_" % seed
+        assert digest(logits, p, lab, td, ls) == str(g[k + "inputs_sha256"]), "input generator drifted"
+
+        def sample(a):
+            return make_golden.layer_sample(a, seed)
+        np.testing.assert_allclose(g[k + "seed_loss"], loss_oracle.balanced_seed_loss(p, lab), rtol=1e-12)
+        np.testing.assert_allclose(g[k + "seed_grad"], sample(loss_oracle.balanced_seed_loss_grad(p, lab)),
+                                   rtol=1e-12, atol=1e-15)
+        np.testing.assert_allclose(g[k + "softmax_probs"], sample(loss_oracle.softmax_layer_forward(logits)), rtol=1e-12)
+        np.testing.assert_allclose(g[k + "softmax_grad"], sample(loss_oracle.softmax_layer_backward(logits, td)),
+                                   rtol=1e-10, atol=1e-15)
+        np.testing.assert_allclose(g[k + "constrain_loss"], loss_oracle.constrain_loss(p, ls), rtol=1e-12)
         w0, w1 = loss_oracle.constrain_loss_grad(p, ls)
-        np.testing.assert_allclose(g0, w0, rtol=1e-12, atol=1e-15)
-        np.testing.assert_allclose(g1, w1, rtol=1e-12, atol=1e-15)
+        np.testing.assert_allclose(g[k + "constrain_g0"], sample(w0), rtol=1e-12, atol=1e-15)
+        np.testing.assert_allclose(g[k + "constrain_g1"], sample(w1), rtol=1e-12, atol=1e-15)
